@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""bench.py -- headline benchmark of the B200 DEFLATE engine (contract: see the task statement).
+"""bench.py -- headline benchmark of the B200 DEFLATE engine: prints one JSON line.
 
 metric  : deflate level-6 GiB/s of raw input on silesia-small.tar (BASELINE.json), zlib wrapper, windowBits 15,
           one deflate(Z_FINISH)-equivalent call per stream -- configs[1].
@@ -10,6 +10,9 @@ e2e     : the same job through the zlib C ABI (compress2) with pinned HOST buffe
 roofline: k_match (the dominant kernel): algorithmic bytes = the raw input each full launch must read once.
 --impl reference : the reference's CPU implementation of the path (the oracle restatement -- zlib-rs itself cannot
           be built here, see DESIGN.md) on the host cores, same workload.
+--dump-outputs DIR : after the timed steps, what the last timed step handed its caller -- the compressed stream as
+          DIR/compressed.npy (one float32 per byte) and its adler32 as DIR/adler32.npy (float64) -- so that two builds can be
+          compared output for output (the input is the same file on every run).
 """
 import argparse
 import ctypes
@@ -44,17 +47,18 @@ def oracle_compress_fn():
     the tests use.  Returns (compress(data, level) -> (rc, bytes), flags description)."""
     if "fn" in _oracle:
         return _oracle["fn"], _oracle["flags"]
-    import hashlib
+    import shutil
+    import tempfile
     import oracle_lib as O
     fn, flags = O.compress, ORACLE_FLAGS["portable"]
     try:
-        model = [l for l in open("/proc/cpuinfo") if l.startswith(("model name", "flags"))][:2]
-        tag = hashlib.sha1("".join(model).encode()).hexdigest()[:10]
-        so = os.path.join(ROOT, "oracle", "_build", "libzoracle_native_%s.so" % tag)
-        if not os.path.exists(so):
-            subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "native", "NATIVE_TAG=" + tag], stdout=subprocess.DEVNULL,
-                                  stderr=subprocess.DEVNULL)
-        L = ctypes.CDLL(so)
+        tmp = tempfile.mkdtemp(prefix="zoracle_native_")  # built per run outside the tree, which may be read-only
+        try:
+            subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "native", "NATIVE_DIR=" + tmp],
+                                  stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+            L = ctypes.CDLL(os.path.join(tmp, "libzoracle_native_host.so"))
+        finally:
+            shutil.rmtree(tmp, ignore_errors=True)
         sz = ctypes.c_size_t
         L.zo_compress_ex.argtypes = [ctypes.c_char_p, ctypes.POINTER(sz), ctypes.c_char_p, sz] + [ctypes.c_int] * 5
 
@@ -88,6 +92,14 @@ def workload(n_streams):
     """config.workload, the same string in both arms."""
     return ("deflate level 6, windowBits 15, memLevel 8, default strategy; %d x silesia-small.tar (15736320 B each), "
             "one compress2 / deflate(Z_FINISH) per stream" % n_streams)
+
+
+def dump_outputs(d, compressed, adler):
+    """--dump-outputs: the compressed stream (one float32 per byte, 25 MiB for silesia-small.tar at level 6) and its adler32."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "compressed.npy"), np.frombuffer(bytes(compressed), dtype=np.uint8).astype(np.float32))
+    np.save(os.path.join(d, "adler32.npy"), np.array([adler], dtype=np.float64))
 
 
 def cpu_sample(tar, reps=2):
@@ -155,15 +167,17 @@ def run_reference(args):
     def one(_):
         rc, out = comp(tar, 6)  # ctypes releases the GIL
         assert rc == 0
-        return len(out)
+        return out
 
     with ThreadPoolExecutor(max_workers=threads) as ex:
         for _ in range(args.warmup):
             list(ex.map(one, range(n_streams)))
         t0 = time.perf_counter()
         for _ in range(args.steps):
-            list(ex.map(one, range(n_streams)))
+            outs = list(ex.map(one, range(n_streams)))
         dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outs[0], int.from_bytes(outs[0][-4:], "big"))  # a zlib stream ends with its adler32
     value = n_streams * len(tar) / dt / GIB
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": "GiB/s", "n_gpus": args.gpus, "steps": args.steps,
@@ -188,7 +202,10 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -282,6 +299,8 @@ def main():
     if dist:
         dist.barrier()
     wall_ms = (time.perf_counter() - t0) * 1e3
+    if args.dump_outputs and rank == 0:  # out_t is reused below, so the last timed step's stream is read back now
+        dump_outputs(args.dump_outputs, out_t[: int(res.out_bytes)].cpu().numpy(), int(res.check))
     ms_per_step = dev_ms / K
     if dist:
         t = torch.tensor([ms_per_step], device=dev)

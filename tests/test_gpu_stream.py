@@ -445,12 +445,12 @@ def test_mixed_flush_sequence_and_deflate_prime():
 
 
 def test_reference_zpipe_binary_round_trip(tmp_path):
-    """The reference's zpipe.c, built unchanged against this library by tests/test_abi_cpu.py (in the build container), compresses and
+    """The reference's zpipe.c, built unchanged against this library by build() (oracle/_ref/zpipe_ref), compresses and
     decompresses a file of several MiB through 16 KiB deflate()/inflate() calls."""
     import subprocess
-    exe = os.path.join(HERE, "c_client", "_build", "zpipe_ref")
+    exe = os.path.join(os.path.dirname(HERE), "oracle", "_ref", "zpipe_ref")
     if not os.path.exists(exe):
-        pytest.skip("zpipe_ref was not built (reference tree absent at build time)")
+        pytest.skip("oracle/_ref/zpipe_ref was not built (no zlib-rs source tree at build time)")
     d = silesia_tar()[: 5 << 20]
     env = dict(os.environ, LD_LIBRARY_PATH=os.path.join(os.path.dirname(HERE), "zlib_rs_b200"))
     z = subprocess.run([exe], input=d, capture_output=True, timeout=600, env=env)
